@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the north-star hot path (rollout-collect -> buffer -> learn()) on B200.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config NAME]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--config NAME] [--dump-outputs DIR]
 
 `--config` selects one of BASELINE.json's configurations; the default (what the driver runs) is configs[1]:
 
@@ -59,7 +59,12 @@ def parse():
     ap.add_argument("--epochs", type=int, default=None)
     ap.add_argument("--buffer", type=int, default=None)
     ap.add_argument("--rounds", type=int, default=None)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    return args
 
 
 def host_cores():
@@ -110,6 +115,39 @@ class ClockSampler:
                     reasons.add(n)
         return {"sm_mhz": sm[len(sm) // 2] if sm else None, "sm_max_mhz": max(mx) if mx else None,
                 "reasons": sorted(reasons), "samples": len(sm)}
+
+
+DUMP_MAX_ELEMS = 1 << 20                # per array: 4 MB in float32, 8 MB in float64
+DUMP_MAX_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays, result):
+    """Writes each tensor of `arrays` and each number of `result` (as `result.<key>`) to out_dir/<name>.npy: floating
+    data as float32, integers and scalars as float64.  An array of more than DUMP_MAX_ELEMS elements is replaced by the
+    same seeded sample of that many of its elements (flattened, ascending index) on every run, so that two builds given
+    the same arguments can be compared file by file."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    out = {}
+    for name, t in arrays.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > DUMP_MAX_ELEMS:
+            idx = np.sort(np.random.RandomState(0).randint(0, flat.numel(), DUMP_MAX_ELEMS))
+            flat = flat[torch.from_numpy(idx).to(flat.device)]
+            a = flat.cpu().numpy()
+        else:
+            a = flat.cpu().numpy().reshape(tuple(t.shape))
+        out[name] = a.astype(np.float32 if a.dtype.kind == "f" else np.float64)
+    for k, v in result.items():
+        if isinstance(v, (bool, int, float, np.number)):
+            out[f"result.{k}"] = np.asarray(v, dtype=np.float64)
+    total = sum(a.nbytes for a in out.values())
+    if total > DUMP_MAX_BYTES:
+        raise ValueError(f"--dump-outputs: {total} bytes exceed the {DUMP_MAX_BYTES}-byte budget")
+    for name, a in out.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+    return total
 
 
 def load_peaks():
@@ -194,6 +232,13 @@ class PPOWorkload:
         self.step_no += self.T
         self.agent.learning_rate_decay(self.step_no)
         return res
+
+    def outputs(self):
+        """What the last step handed back: the rollout collect() returned and the network learn() left."""
+        ro = self.col.rollout
+        out = {f"rollout.{k}": getattr(ro, k) for k in ("state", "action", "reward", "done", "last_next_state")}
+        out.update({f"network.{k}": v for k, v in self.agent.network.p.items()})
+        return out
 
     def env_steps_per_step(self):
         return self.n_envs * self.T * self.world
@@ -470,6 +515,9 @@ class ReplayWorkload:
             res = r or res
         return res
 
+    def outputs(self):
+        return {f"network.{k}": v for k, v in self.agent.network.p.items()}
+
     def env_steps_per_step(self):
         return self.n_actors * self.update_period * self.rounds * self.world
 
@@ -735,6 +783,13 @@ class ACWorkload:
             res = r or res
         return res
 
+    def outputs(self):
+        out = {f"actor.{k}": v for k, v in self.agent.actor.p.items()}
+        for i, c in enumerate(self.agent.critics):
+            out.update({f"critic{i + 1}.{k}": v for k, v in c.p.items()})
+        out["log_alpha"] = self.agent.log_alpha.flat[:1]
+        return out
+
     def env_steps_per_step(self):
         return self.n_actors * self.update_period * self.rounds * self.world
 
@@ -935,6 +990,10 @@ def main():
 
     torch.cuda.set_device(local_rank)
     dev = torch.device("cuda", local_rank)
+    # network initialisation, minibatch permutations and replay sampling draw from the global generators: seeding them
+    # gives every run with the same arguments the same inputs
+    torch.manual_seed(0)
+    np.random.seed(0)
     if world > 1:
         dist.init_process_group("nccl", device_id=dev)
     trace_all = os.environ.get("JB_BENCH_TRACE", "0") == "1"
@@ -969,6 +1028,9 @@ def main():
     torch.cuda.synchronize()
     ms = e0.elapsed_time(e1)
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        n = dump_outputs(args.dump_outputs, wl.outputs(), res)
+        log(f"outputs of the last timed step ({n} bytes) written to {args.dump_outputs}")
     t = torch.tensor([ms], dtype=torch.float64, device=dev)
     if world > 1:
         dist.barrier()

@@ -196,3 +196,24 @@ def test_public_headers_are_plain_c99(tmp_path):
     import ctypes
     from jorldy_b200.core.agent.ppo_fused import FusedArgs
     assert size == ctypes.sizeof(FusedArgs)
+
+
+def test_bench_dump_outputs_files(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: floating data as float32, integers and scalar results as float64, an array above
+    DUMP_MAX_ELEMS replaced by the same seeded sample on every call, and the byte budget enforced."""
+    import bench
+    arrays = {"net.big": torch.arange(bench.DUMP_MAX_ELEMS + 5, dtype=torch.float32),
+              "rollout.action": torch.arange(6, dtype=torch.int32).view(2, 3)}
+    result = {"loss": 0.5, "note": "not a number"}
+    for d in ("d1", "d2"):
+        bench.dump_outputs(str(tmp_path / d), arrays, result)
+    assert sorted(os.listdir(tmp_path / "d1")) == ["net.big.npy", "result.loss.npy", "rollout.action.npy"]
+    big1, big2 = np.load(tmp_path / "d1" / "net.big.npy"), np.load(tmp_path / "d2" / "net.big.npy")
+    assert big1.dtype == np.float32 and big1.shape == (bench.DUMP_MAX_ELEMS,) and np.array_equal(big1, big2)
+    assert np.all(np.diff(big1) >= 0)
+    act = np.load(tmp_path / "d1" / "rollout.action.npy")
+    assert act.dtype == np.float64 and np.array_equal(act, np.arange(6).reshape(2, 3))
+    assert np.load(tmp_path / "d1" / "result.loss.npy") == 0.5
+    monkeypatch.setattr(bench, "DUMP_MAX_BYTES", 1024)
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "d3"), arrays, result)
