@@ -69,6 +69,33 @@ JB_API int
 jb_replay_gather(const void* ring, const int64_t* idx, int n, long long row_bytes, void* batch, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
+ * Frame-deduplicated replay (csrc/frame_replay.cu) — replay_buffer.py:16-31 (ring write / sample), base.py:42-56
+ * (stack_transition), per_buffer.py:95-96 (PER gather) for uint8 frame-stack fields [S, H, W], H*W % 16 == 0.
+ * Each distinct frame is stored once: frames [F, frame_bytes] holds frame id i at row i % F; ref [nf, capacity, S] int64
+ * the ids of each slot's stacks, min_ref [capacity] the oldest of them (INT64_MAX when empty);
+ * ctl int64[4] = {next id, first id of the last store, its new frames, sticky overflow flag}.
+ * host_fields is a HOST array of nf (<= 4) device pointers, field f = [n, S, frame_bytes]; row t*N + r is actor r at step t.
+ *   jb_frame_plan    hashes u64[n*nf*S] (scratch); per actor, in row order: reuse a frame of hist_id/hist_h [N,16] (most
+ *                    recently used first, byte-compared, id >= next id - F) or take the actor's next new frame.
+ *                    codes [n*nf*S] = pool id or -(j+1), newsrc [n*nf*S] = batch frame of new frame j of actor r at r*(n/N)*nf*S + j, counts [N]
+ *   jb_frame_assign  offs [N] = exclusive scan of counts (ids actor-major), ctl update, and the overflow check over the
+ *                    min_ref of the slots outside [start, start+n) (mod capacity) and the n_codes reused ids in codes
+ *   jb_frame_commit  new frames -> frames (not while the flag is set), ref / min_ref of the rows written, history -> ids
+ *   jb_frame_gather  out [B, S, frame_bytes] = frames[ref[idx[b], s] % F] for one field's ref table
+ * ------------------------------------------------------------------------------------------- */
+JB_API int jb_frame_plan(const void* host_fields, int nf, int n, int N, int S, long long frame_bytes, const uint8_t* frames,
+                         int64_t F, uint64_t* hashes, const int64_t* ctl, int64_t* hist_id, uint64_t* hist_h, int64_t* codes,
+                         int64_t* newsrc, int64_t* counts, void* stream);
+JB_API int jb_frame_assign(const int64_t* counts, int N, int64_t F, const int64_t* min_ref, int64_t capacity, int64_t start,
+                           int64_t n, const int64_t* codes, int64_t n_codes, int64_t* offs, int64_t* ctl, void* stream);
+JB_API int jb_frame_commit(const void* host_fields, int nf, int n, int N, int S, long long frame_bytes, uint8_t* frames,
+                           int64_t F, const int64_t* ctl, const int64_t* counts, const int64_t* offs, const int64_t* newsrc,
+                           const int64_t* codes, int64_t* ref, int64_t* min_ref, int64_t capacity, int64_t start,
+                           int64_t* hist_id, void* stream);
+JB_API int jb_frame_gather(const uint8_t* frames, int64_t F, long long frame_bytes, const int64_t* ref, int S,
+                           const int64_t* idx, int B, uint8_t* out, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
  * PER sum-tree — jorldy/core/buffer/per_buffer.py:19-101.  tree is f64[2*capacity-1].
  * ------------------------------------------------------------------------------------------- */
 JB_API int jb_per_update(double* tree, int64_t capacity, const int64_t* tree_idx, int64_t first_idx,

@@ -12,7 +12,7 @@ from collections import deque
 import numpy as np
 import torch
 
-from ..buffer import PERBuffer, ReplayBuffer
+from ..buffer import FramePERBuffer, FrameReplayBuffer, PERBuffer, ReplayBuffer
 from ..dev import C, ptr, require_cuda, stream_ptr
 from ..network import Network
 from ..optimizer import Optimizer
@@ -35,7 +35,7 @@ class DQN(BaseAgent):
                  network="discrete_q_network", head="mlp", gamma=0.99, epsilon_init=1.0, epsilon_min=0.1,
                  epsilon_eval=0.0, explore_ratio=0.1, buffer_size=50000, batch_size=64, start_train_step=2000,
                  target_update_period=500, device=None, run_step=1e6, num_workers=1, lr_decay=True, seed=0,
-                 **kwargs):
+                 frame_replay=False, **kwargs):
         self.device = require_cuda(device)
         self.state_size, self.action_size = state_size, action_size
         self.action_type = "discrete"
@@ -49,7 +49,8 @@ class DQN(BaseAgent):
         self.explore_step = run_step * explore_ratio
         self.epsilon_delta = (epsilon_init - epsilon_min) / self.explore_step
         self.buffer_size = buffer_size
-        self.memory = ReplayBuffer(buffer_size, device=self.device)
+        self.frame_replay = frame_replay   # store uint8 frame stacks once per frame (core/buffer/frame_replay.py)
+        self.memory = (FrameReplayBuffer if frame_replay else ReplayBuffer)(buffer_size, device=self.device)
         self.batch_size = batch_size
         self.start_train_step = start_train_step
         self.target_update_stamp = 0
@@ -155,10 +156,20 @@ class DQN(BaseAgent):
         self.num_learn += 1
         return prio
 
+    def _stats_host(self, stats):
+        """stats.cpu().numpy(): learn()'s device->host read.  With the frame replay the same copy carries its overflow
+        flag, so a result computed from a stack the pool could no longer hold raises instead of being returned."""
+        flag = getattr(self.memory, "overflow_flag", None)
+        if flag is None:
+            return stats.cpu().numpy()
+        both = torch.cat([stats.to(torch.float64), flag.to(torch.float64)]).cpu().numpy()
+        self.memory.raise_if_overflow(both[-1] != 0)
+        return both[:-1].astype(np.float32)
+
     def learn(self):
         batch, _, _, _ = self._sample()
         self._learn_batch(batch)
-        st = self._stats[:2].cpu().numpy()
+        st = self._stats_host(self._stats[:2])
         return {"loss": float(st[0]), "epsilon": self.epsilon, "max_Q": float(st[1])}
 
     def update_target(self):
@@ -248,7 +259,8 @@ class PER(DQN):
 
     def __init__(self, alpha=0.6, beta=0.4, learn_period=16, uniform_sample_prob=1e-3, run_step=1e6, **kwargs):
         super().__init__(run_step=run_step, **kwargs)
-        self.memory = PERBuffer(self.buffer_size, uniform_sample_prob, device=self.device, seed=self.seed)
+        self.memory = (FramePERBuffer if self.frame_replay else PERBuffer)(self.buffer_size, uniform_sample_prob,
+                                                                           device=self.device, seed=self.seed)
         self.alpha = alpha
         self.beta = beta
         self.beta_add = (1 - beta) / run_step
@@ -263,7 +275,7 @@ class PER(DQN):
         return self.memory.sample_device(self.beta, self.batch_size, u_a, u_b)
 
     def _per_result(self, stats_per):
-        st = self._stats[:2].cpu().numpy()
+        st = self._stats_host(self._stats[:2])
         sp = stats_per.cpu().numpy()
         return float(st[0]), float(st[1]), float(sp[0]), float(sp[1])
 
@@ -336,7 +348,7 @@ class Noisy(DQN):
     def learn(self):
         batch, _, _, _ = self._sample()
         self._learn_batch(batch)
-        st = self._stats[:2].cpu().numpy()
+        st = self._stats_host(self._stats[:2])
         s1, s2 = self.network.get_sig_w_mean()
         return {"loss": float(st[0]), "max_Q": float(st[1]), "sig_w1": float(s1.item()), "sig_w2": float(s2.item())}
 
@@ -416,7 +428,7 @@ class C51(DQN, _Distributional):
     def learn(self):
         batch, _, _, _ = self._sample()
         self._dist_learn(batch, None, 0, [None, None, None])
-        st = self._stats.cpu().numpy()
+        st = self._stats_host(self._stats)
         return {"loss": float(st[0]), "epsilon": self.epsilon, "max_Q": float(st[1]), "max_logit": float(st[2]),
                 "min_logit": float(st[3])}
 
@@ -426,13 +438,14 @@ class Rainbow(PER, _Distributional):
                  optim_config={"name": "adam"}, gamma=0.99, buffer_size=50000, batch_size=64, start_train_step=2000,
                  target_update_period=500, run_step=1e6, lr_decay=True, n_step=4, alpha=0.6, beta=0.4, learn_period=4,
                  uniform_sample_prob=1e-3, noise_type="factorized", v_min=-10, v_max=10, num_support=51, device=None,
-                 seed=0, **kwargs):
+                 seed=0, frame_replay=False, **kwargs):
         self._noise_type, self._num_support = noise_type, num_support
         super().__init__(alpha=alpha, beta=beta, learn_period=learn_period, uniform_sample_prob=uniform_sample_prob,
                          run_step=run_step, state_size=state_size, action_size=action_size, hidden_size=hidden_size,
                          network=network, head=head, optim_config=optim_config, gamma=gamma, buffer_size=buffer_size,
                          batch_size=batch_size, start_train_step=start_train_step,
-                         target_update_period=target_update_period, lr_decay=lr_decay, device=device, seed=seed)
+                         target_update_period=target_update_period, lr_decay=lr_decay, device=device, seed=seed,
+                         frame_replay=frame_replay)
         self.n_step = n_step
         self.tmp_buffer = deque(maxlen=n_step)
         self._setup_support(v_min, v_max, num_support)
@@ -461,7 +474,7 @@ class Rainbow(PER, _Distributional):
         noise = self._inject_noise or [None, None, None]
         prio = self._dist_learn(batch, weights, 1, noise)
         self.memory.update_priorities(indices, prio)
-        st = self._stats.cpu().numpy()
+        st = self._stats_host(self._stats)
         sp = stats_per.cpu().numpy()
         return {"loss": float(st[0]), "beta": self.beta, "max_Q": float(st[1]), "max_logit": float(st[2]),
                 "min_logit": float(st[3]), "sampled_p": float(sp[0]), "mean_p": float(sp[1])}
