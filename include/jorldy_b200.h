@@ -176,6 +176,10 @@ JB_API int jb_env_frames_step(uint8_t* obs, int64_t* fcount, float* score, uint8
  * CNN head lowering — jorldy/core/network/head.py:21-61 (im2col / col2im around jb_gemm).
  * ------------------------------------------------------------------------------------------- */
 JB_API int jb_im2col_u8(const uint8_t* x, int B, int C, int H, int W, int KH, int KW, int S, float* col, void* stream);
+/* Same, with output row b read from input row idx[b] (int32, < rows of x; NULL: row b): gathers a minibatch of
+ * uint8 [rows, C, H, W] stacks inside conv1's im2col.  jb_im2col_u8 is this call with idx = NULL. */
+JB_API int jb_im2col_u8_rows(const uint8_t* x, const int32_t* idx, int B, int C, int H, int W, int KH, int KW, int S,
+                             float* col, void* stream);
 JB_API int jb_im2col_nhwc(const float* x, int B, int C, int H, int W, int KH, int KW, int S, float* col, void* stream);
 JB_API int jb_col2im_nhwc(const float* dcol, int B, int C, int H, int W, int KH, int KW, int S, const float* relu_act,
                           float* dx, void* stream);

@@ -77,6 +77,13 @@ def _ppo_config(env):
                                eval_iteration=10, record=True, record_period=500000, distributed_batch_size=2048,
                                update_period=2048, num_workers=32))
     a.update(batch_size=32, n_step=128, n_epoch=3, use_standardization=True)
+    if env == "atari":
+        # Shaped after the reference's config/ppo/atari.py: the cartpole PPO agent keys plus head="cnn", with the Atari
+        # env and train dicts the value agents use.  Not checked line by line against that file.
+        a.update(network="discrete_policy_value", head="cnn")
+        return dict(env=dict(_ATARI_ENV), agent=a, optim=dict(name="adam", lr=2.5e-4),
+                    train=dict(_TRAIN_ATARI, run_step=30000000, distributed_batch_size=1024, update_period=128,
+                               num_workers=32))
     if env == "pendulum":
         a.update(network="continuous_policy_value")
         env_d = dict(name="pendulum", render=False)
@@ -142,7 +149,7 @@ def available():
         out += [f"config.{ag}.{e}" for e in envs]
     for ag in list(_VALUE_AGENTS) + ["ape_x"]:
         out += [f"config.{ag}.{e}" for e in ("cartpole", "mountaincar", "atari")]
-    out += [f"config.ppo.{e}" for e in ("cartpole", "mountaincar", "pendulum", "mujoco")]
+    out += [f"config.ppo.{e}" for e in ("cartpole", "mountaincar", "pendulum", "mujoco", "atari")]
     return out
 
 
@@ -155,7 +162,7 @@ def load(config_path):
         d = _value_config(agent, env)
     elif agent == "ape_x" and env in ("cartpole", "mountaincar", "atari"):
         d = _ape_x_config(env)
-    elif agent == "ppo" and env in ("cartpole", "mountaincar", "pendulum", "mujoco"):
+    elif agent == "ppo" and env in ("cartpole", "mountaincar", "pendulum", "mujoco", "atari"):
         d = _ppo_config(env)
     elif agent in _AC_ENVS and env in _AC_ENVS[agent]:
         d = _ac_config(agent, env)

@@ -58,6 +58,10 @@ class PPO(BaseAgent):
         self.state_size, self.action_size = state_size, action_size
         self.network = Network(network, state_size, action_size, D_hidden=hidden_size, head=head,
                                device=self.device)
+        # device row layout of a state: uint8 [C, H, W] frame stacks for the CNN head (it scales by 1/255 itself),
+        # f32 [D] vectors for the MLP head
+        h = self.network.head
+        self._row_shape, self._row_dtype = ((h.D_in, torch.uint8) if h.kind == "cnn" else ((h.D_in,), torch.float32))
         optim_config = dict(optim_config)
         self.optimizer = Optimizer(**optim_config, params=self.network.parameters())
 
@@ -100,7 +104,7 @@ class PPO(BaseAgent):
         return self.action_type == "continuous"
 
     def act_device(self, state, training=True, noise=None):
-        """state: [N, D] f32 device tensor -> action device tensor ([N] int64 / [N, A] f32)."""
+        """state: [N, D] f32 / [N, C, H, W] uint8 device tensor -> action device tensor ([N] int64 / [N, A] f32)."""
         net = self.network
         M = state.shape[0]
         out = net._buf("act.out", (M, net.nout))
@@ -119,11 +123,17 @@ class PPO(BaseAgent):
                                   0, ptr(row_ctr), int(not training), ptr(action), stream_ptr())
         return action
 
+    def _state_rows(self, state):
+        """Host or device states -> device rows in the network's input layout (see _row_shape)."""
+        if self._row_dtype == torch.uint8:
+            return torch.as_tensor(state, device=self.device).reshape(-1, *self._row_shape)
+        s = self.as_tensor(state)
+        return s.view(s.shape[0], -1)
+
     @torch.no_grad()
     def act(self, state, training=True):
         self.network.train(training)
-        s = self.as_tensor(state)
-        action = self.act_device(s.view(s.shape[0], -1), training)
+        action = self.act_device(self._state_rows(state), training)
         a = action.cpu().numpy()
         return {"action": a.reshape(a.shape[0], -1)}
 
@@ -144,6 +154,11 @@ class PPO(BaseAgent):
         self.optimizer.step(max_norm=self.clip_grad_norm)
 
     LAUNCHES_PER_MINIBATCH = 13   # take + in_fwd + gemm + heads + loss + finalize + 2 heads bwd + 3 gemm + sumsq + adam
+
+    def _launches_per_minibatch(self, B):
+        """LAUNCHES_PER_MINIBATCH with the input head's own forward / backward kernels (1 + 1 for the MLP head)."""
+        h = self.network.head
+        return self.LAUNCHES_PER_MINIBATCH - 2 + h.fwd_launches + h.bwd_launches(B)
 
     def _graph_for(self, st, B):
         """CUDA graph of GRAPH_CHUNK minibatch steps reading indices through the device cursor."""
@@ -260,10 +275,13 @@ class PPO(BaseAgent):
             if tail:
                 self._minibatch_step(st, st["perm"][n_full * B:], tail)
             n_steps += n_full + (1 if tail else 0)
-        self.n_launches = (self.n_epoch * (1 + (self.LAUNCHES_PER_MINIBATCH if tail else 0)) if use_fused
-                           else n_steps * self.LAUNCHES_PER_MINIBATCH)
-        n_chunks = (NT + 16383) // 16384
-        self.n_prepass_launches = 3 * n_chunks + 1 + 3 + 1      # forward chunks + prepass + V(s') + gae
+        per_tail = self._launches_per_minibatch(tail) if tail else 0
+        self.n_launches = (self.n_epoch * (1 + per_tail) if use_fused
+                           else self.n_epoch * (n_full * self._launches_per_minibatch(B) + per_tail))
+        per_pass, rows = net.head.fwd_launches + 2, net.head.max_rows     # head + gemm + heads per inference chunk
+        n_next = NT if next_state is not None else N
+        # forward chunks + prepass + V(s') chunks + gae
+        self.n_prepass_launches = per_pass * -(-NT // rows) + 1 + per_pass * -(-n_next // rows) + 1
 
         acc = torch.cat([self._acc[:6], mean_ret.view(1), self._acc[7:8]]).cpu().numpy()     # ONE device->host read
         if acc[7] != 0.0:
@@ -295,14 +313,14 @@ class PPO(BaseAgent):
         hin = getattr(self, "_host_in", None)
         if hin is None or hin["n"] != n:
             hin = {"n": n,
-                   "state": torch.empty(n, int(np.prod(np.shape(tr["state"])[1:])), device=dev),
-                   "next_state": torch.empty(n, int(np.prod(np.shape(tr["state"])[1:])), device=dev),
+                   "state": torch.empty(n, *self._row_shape, dtype=self._row_dtype, device=dev),
+                   "next_state": torch.empty(n, *self._row_shape, dtype=self._row_dtype, device=dev),
                    "reward": torch.empty(n, device=dev), "done": torch.empty(n, device=dev),
                    "action": (torch.empty(n, self.action_size, device=dev) if self.continuous
                               else torch.empty(n, dtype=torch.int32, device=dev))}
             self._host_in = hin
-        hin["state"].copy_(torch.as_tensor(tr["state"], dtype=torch.float32, device=dev).reshape(n, -1))
-        hin["next_state"].copy_(torch.as_tensor(tr["next_state"], dtype=torch.float32, device=dev).reshape(n, -1))
+        hin["state"].copy_(self._state_rows(tr["state"]))
+        hin["next_state"].copy_(self._state_rows(tr["next_state"]))
         hin["reward"].copy_(torch.as_tensor(tr["reward"], dtype=torch.float32, device=dev).reshape(-1))
         hin["done"].copy_(torch.as_tensor(tr["done"], dtype=torch.float32, device=dev).reshape(-1))
         hin["action"].copy_(self._action_to_device(tr["action"]))
@@ -311,7 +329,7 @@ class PPO(BaseAgent):
     def learn_rollout(self, rollout):
         """Resident path: `rollout` is a DeviceRollout filled by the batched collect loop."""
         N, T = rollout.N, rollout.T
-        res = self._learn_tensors(rollout.state.view(N * T, -1), rollout.action.view(N * T, -1) if self.continuous
+        res = self._learn_tensors(rollout.state.view(N * T, *self._row_shape), rollout.action.view(N * T, -1) if self.continuous
                                   else rollout.action.view(N * T), rollout.reward.view(N * T),
                                   rollout.done.view(N * T), last_next_state=rollout.last_next_state)
         rollout.clear()

@@ -48,14 +48,20 @@ class DeviceRollout:
         dev = require_cuda(device)
         N, T = num_envs, n_step
         self.N, self.T, self.device = N, T, dev
-        self.state = torch.zeros(N, T, state_size, dtype=torch.float32, device=dev)
+        # a shaped state is a uint8 frame stack, kept as the env produces it (4x84x84: 28 224 B a row instead of 4x that
+        # as f32); a vector state is f32
+        if isinstance(state_size, (list, tuple)):
+            shape, sdtype = tuple(state_size), torch.uint8
+        else:
+            shape, sdtype = (state_size,), torch.float32
+        self.state = torch.zeros(N, T, *shape, dtype=sdtype, device=dev)
         if action_type == "discrete":
             self.action = torch.zeros(N, T, dtype=torch.int32, device=dev)
         else:
             self.action = torch.zeros(N, T, action_size, dtype=torch.float32, device=dev)
         self.reward = torch.zeros(N, T, dtype=torch.float32, device=dev)
         self.done = torch.zeros(N, T, dtype=torch.float32, device=dev)
-        self.last_next_state = torch.zeros(N, state_size, dtype=torch.float32, device=dev)
+        self.last_next_state = torch.zeros(N, *shape, dtype=sdtype, device=dev)
         self.t = 0
 
     def write(self, state, action, reward, done, next_state):

@@ -18,9 +18,10 @@ class RolloutCollector:
                                      device=agent.device)
         self.use_cuda_graph = use_cuda_graph
         self._graph = None
-        # kernels of OUR library per env step: mlp_in_fwd + gemm + heads_fwd + act + env_step (the
-        # rollout-row copies are torch plumbing and not counted)
-        self.launches_per_collect = 5 * self.T
+        # kernels of OUR library per env step: input head + gemm + heads_fwd per inference chunk of envs (one chunk of
+        # mlp_in_fwd for the MLP head), then act + env_step (the rollout-row copies are torch plumbing and not counted)
+        h = agent.network.head
+        self.launches_per_collect = ((h.fwd_launches + 2) * -(-env.num_envs // h.max_rows) + 2) * self.T
         env.reset_device()
 
     def _collect_eager(self):

@@ -13,6 +13,10 @@ from .base import init_gain, orthogonal_
 class MLPHead:
     kind = "mlp"
     max_rows = 16384        # inference chunk: activations (2 x 32 MB at H=512) stay L2-resident
+    fwd_launches = 1        # kernels of forward() (launch bookkeeping of the agents and collectors)
+
+    def bwd_launches(self, M):
+        return 1
 
     def __init__(self, D_in, D_hidden=512):
         if not isinstance(D_in, int):
@@ -45,6 +49,7 @@ class CNNHead:
     """head.py:21-61.  Input: uint8 [rows, C, H, W] (NCHW, as the env / replay produce it)."""
     kind = "cnn"
     max_rows = 256          # inference chunk: the first im2col buffer is 400 KB per row
+    fwd_launches = 7        # 3 x (im2col + gemm) + flatten
 
     def __init__(self, D_in, D_hidden=512):
         C, H, W = D_in
@@ -71,18 +76,20 @@ class CNNHead:
             p[f"head.{name}.bias"].zero_()
 
     def forward(self, net, x, idx, M, tag, save):
-        if idx is not None:
-            x = x.index_select(0, idx.to(torch.int64))
-        if x.dtype != torch.uint8:
-            x = x.to(torch.uint8)
-        x = x.contiguous()
+        """x: contiguous uint8 [rows, C, H, W] (all rows if idx is None else gathered by idx[M] int32 inside conv1's
+        im2col)."""
+        if x.dtype != torch.uint8 or not x.is_contiguous() or tuple(x.shape[1:]) != self.D_in:
+            raise ValueError(f"cnn head expects a contiguous uint8 [rows, {', '.join(map(str, self.D_in))}] tensor, "
+                             f"got {x.dtype} {tuple(x.shape)}{'' if x.is_contiguous() else ' (non-contiguous)'}")
+        if idx is not None and (idx.dtype != torch.int32 or not idx.is_contiguous()):
+            raise ValueError(f"cnn head expects contiguous int32 row indices, got {idx.dtype}")
         s = stream_ptr()
         cur = None
         for li, (name, ci, co, k, st, (ih, iw), (oh, ow)) in enumerate(self.layers):
             K = ci * k * k
             col = net._buf(f"{tag}head.col{li}", (M * oh * ow, K))
             if li == 0:
-                C.jb_im2col_u8(ptr(x), M, ci, ih, iw, k, k, st, ptr(col), s)
+                C.jb_im2col_u8_rows(ptr(x), ptr(idx), M, ci, ih, iw, k, k, st, ptr(col), s)
             else:
                 C.jb_im2col_nhwc(ptr(cur), M, ci, ih, iw, k, k, st, ptr(col), s)
             y = net._buf(f"{tag}head.y{li}", (M * oh * ow, co))
@@ -93,6 +100,17 @@ class CNNHead:
         feat = net._buf(tag + "head.h", (M, self.D_head_out))
         C.jb_nhwc_to_nchw(ptr(cur), M, P, 64, ptr(feat), s)
         return feat
+
+    def _dw_splits(self, li, M):
+        # conv weight gradients are [co, ci k k] = a few 32 x 32 tiles contracted over M * oh * ow rows: split the
+        # contraction over the grid (148 SMs) and fold the partials in a fixed order
+        _, ci, co, k, _, _, (oh, ow) = self.layers[li]
+        tiles = ((ci * k * k + 31) // 32) * ((co + 31) // 32)
+        return min(64, max(1, 296 // tiles), max(1, M * oh * ow // 512))
+
+    def bwd_launches(self, M):
+        """unflatten + per layer dW (split-K: gemm + 2 folds) + dcol and col2im for conv3 and conv2."""
+        return 1 + sum(3 if self._dw_splits(li, M) > 1 else 1 for li in range(3)) + 2 * 2
 
     def backward(self, net, dfeat_pre, M, tag):
         """dfeat_pre [M, 64*P] (C,H,W order): gradient w.r.t. conv3's pre-activation (already ReLU-masked)."""
@@ -105,10 +123,7 @@ class CNNHead:
             K = ci * k * k
             Mr = M * oh * ow
             col = net._buf(f"{tag}head.col{li}", (Mr, K))
-            # conv weight gradients are [co, ci k k] = a few 32 x 32 tiles contracted over M * oh * ow rows: split the
-            # contraction over the grid (148 SMs) and fold the partials in a fixed order
-            tiles = ((K + 31) // 32) * ((co + 31) // 32)
-            splits = min(64, max(1, 296 // tiles), max(1, Mr // 512))
+            splits = self._dw_splits(li, M)
             ws = net._buf(f"{tag}head.dwws{li}", (splits * (co * K + co),)) if splits > 1 else None
             C.jb_linear_bwd_dw_splitk(ptr(dy), ptr(col), ptr(net.g[f"head.{name}.weight"]), ptr(net.g[f"head.{name}.bias"]),
                                       Mr, K, co, ptr(ws), splits, s)

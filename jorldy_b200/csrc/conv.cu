@@ -14,9 +14,11 @@
 
 namespace {
 
-// x: [B, C, H, W] uint8 (NCHW, the env/replay layout)  ->  col [B*OH*OW, C*KH*KW] f32, scaled by 1/255
-__global__ void im2col_u8_nchw_kernel(const uint8_t* __restrict__ x, int B, int C, int H, int W, int KH, int KW, int S,
-                                      int OH, int OW, float* __restrict__ col) {
+// x: [rows, C, H, W] uint8 (NCHW, the env/replay/rollout layout)  ->  col [B*OH*OW, C*KH*KW] f32, scaled by 1/255.
+// Output row b reads input row idx[b] (idx NULL: row b), so a minibatch is gathered inside the im2col.  Row byte
+// offsets are 64-bit: a 4x84x84 stack is 28 224 B, so row indices from 76 088 up lie past 2^31 bytes.
+__global__ void im2col_u8_nchw_kernel(const uint8_t* __restrict__ x, const int32_t* __restrict__ idx, int B, int C,
+                                      int H, int W, int KH, int KW, int S, int OH, int OW, float* __restrict__ col) {
   const int K = C * KH * KW;
   const long long total = (long long)B * OH * OW * K;
   for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
@@ -25,15 +27,16 @@ __global__ void im2col_u8_nchw_kernel(const uint8_t* __restrict__ x, int B, int 
     const int ox = (int)(m % OW), oy = (int)((m / OW) % OH), b = (int)(m / ((long long)OW * OH));
     const int kx = k % KW, ky = (k / KW) % KH, c = k / (KW * KH);
     const int iy = oy * S + ky, ix = ox * S + kx;
-    const float v = (float)x[(((size_t)b * C + c) * H + iy) * W + ix];
+    const long long row = idx ? (long long)idx[b] : (long long)b;
+    const float v = (float)x[row * C * H * W + ((size_t)c * H + iy) * W + ix];
     col[e] = v / 255.0f;
   }
 }
 
 // Same, four consecutive kx per thread (KW % 4 == 0, S % 4 == 0, W % 4 == 0: the 8x8 stride-4 first layer): one 4-byte
-// load of the frame row and one 16-byte store of the column row per thread, 32-bit index arithmetic.
-__global__ void im2col_u8_nchw_vec4_kernel(const uint8_t* __restrict__ x, int B, int C, int H, int W, int KH, int KW, int S,
-                                           int OH, int OW, float* __restrict__ col) {
+// load of the frame row and one 16-byte store of the column row per thread, 32-bit index arithmetic inside a row.
+__global__ void im2col_u8_nchw_vec4_kernel(const uint8_t* __restrict__ x, const int32_t* __restrict__ idx, int B, int C,
+                                           int H, int W, int KH, int KW, int S, int OH, int OW, float* __restrict__ col) {
   const int K4 = (C * KH * KW) >> 2, KW4 = KW >> 2;
   const long long total = (long long)B * OH * OW * K4;
   for (long long e = (long long)blockIdx.x * blockDim.x + threadIdx.x; e < total; e += (long long)gridDim.x * blockDim.x) {
@@ -41,7 +44,8 @@ __global__ void im2col_u8_nchw_vec4_kernel(const uint8_t* __restrict__ x, int B,
     const int m = (int)(e / K4);
     const int ox = m % OW, t = m / OW, oy = t % OH, b = t / OH;
     const int kx4 = k4 % KW4, t2 = k4 / KW4, ky = t2 % KH, c = t2 / KH;
-    const uchar4 v = *reinterpret_cast<const uchar4*>(x + (((size_t)b * C + c) * H + oy * S + ky) * W + ox * S + 4 * kx4);
+    const long long row = idx ? (long long)idx[b] : (long long)b;
+    const uchar4 v = *reinterpret_cast<const uchar4*>(x + row * C * H * W + (c * H + oy * S + ky) * W + ox * S + 4 * kx4);
     reinterpret_cast<float4*>(col)[e] = make_float4((float)v.x / 255.0f, (float)v.y / 255.0f, (float)v.z / 255.0f, (float)v.w / 255.0f);
   }
 }
@@ -112,15 +116,23 @@ __global__ void permute_bpc_kernel(const float* __restrict__ x, int B, int P, in
 
 static int conv_grid(long long total) { return jb_grid_for(total, 256 * 4, 8); }
 
-JB_API int jb_im2col_u8(const uint8_t* x, int B, int C, int H, int W, int KH, int KW, int S, float* col, void* stream) {
+JB_API int jb_im2col_u8_rows(const uint8_t* x, const int32_t* idx, int B, int C, int H, int W, int KH, int KW, int S,
+                             float* col, void* stream) {
   if (!x || !col || B <= 0 || C <= 0 || H < KH || W < KW || S <= 0) return JB_ERR_INVALID;
   const int OH = (H - KH) / S + 1, OW = (W - KW) / S + 1;
   const long long total = (long long)B * OH * OW * C * KH * KW;
-  if (KW % 4 == 0 && S % 4 == 0 && W % 4 == 0 && (((uintptr_t)x | (uintptr_t)col) & 15) == 0 && (long long)B * OH * OW < (1ll << 31))
-    im2col_u8_nchw_vec4_kernel<<<conv_grid(total / 4), 256, 0, (cudaStream_t)stream>>>(x, B, C, H, W, KH, KW, S, OH, OW, col);
+  // a gathered row starts where x does modulo 16 only when the row size is a multiple of 16 (4x84x84: 16 x 1 764)
+  const bool rows_aligned = !idx || ((long long)C * H * W) % 16 == 0;
+  if (KW % 4 == 0 && S % 4 == 0 && W % 4 == 0 && (((uintptr_t)x | (uintptr_t)col) & 15) == 0 && rows_aligned &&
+      (long long)B * OH * OW < (1ll << 31))
+    im2col_u8_nchw_vec4_kernel<<<conv_grid(total / 4), 256, 0, (cudaStream_t)stream>>>(x, idx, B, C, H, W, KH, KW, S, OH, OW, col);
   else
-    im2col_u8_nchw_kernel<<<conv_grid(total), 256, 0, (cudaStream_t)stream>>>(x, B, C, H, W, KH, KW, S, OH, OW, col);
+    im2col_u8_nchw_kernel<<<conv_grid(total), 256, 0, (cudaStream_t)stream>>>(x, idx, B, C, H, W, KH, KW, S, OH, OW, col);
   return jb_check_launch();
+}
+
+JB_API int jb_im2col_u8(const uint8_t* x, int B, int C, int H, int W, int KH, int KW, int S, float* col, void* stream) {
+  return jb_im2col_u8_rows(x, nullptr, B, C, H, W, KH, KW, S, col, stream);
 }
 
 JB_API int jb_im2col_nhwc(const float* x, int B, int C, int H, int W, int KH, int KW, int S, float* col, void* stream) {
